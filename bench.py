@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the reduced-order frequency-sweep hot path (BASELINE.json metric: reduced-sweep freq points/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg3|cfg2|cfg5|mid|small]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg3|cfg2|cfg5|mid|small] [--dump-outputs DIR]
 
 One "step" = one pass of the four hot stages over one synthetic batch: orthonormalise the snapshot block
 (CholeskyQR2 + SVD of R), Galerkin-project Ct/Tt/WP, solve every reduced system, evaluate the S-parameters.
@@ -15,6 +15,8 @@ partials all-reduced, Q halo rows exchanged, S-parameters all-gathered.
 ``parity``= the S-parameters of the timed configuration against the CPU restatement of the reference (oracle/);
 ``--impl reference`` times that CPU restatement (numpy/scipy = the library calls the pure-Python reference makes)
 on all host cores of rank 0, each step a bounded sample of the same global workload.
+``--dump-outputs DIR`` writes what the last timed step returned as .npy files: the inputs are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -62,6 +64,9 @@ UNIT = "points/s"
 FP64_PEAK_FALLBACK = 37.05   # TFLOP/s, DMMA m8n8k4 issue loop measured on this pool's B200 in round 1 (profiles/r01_fp64_peaks.jsonl)
 SNAP_BLOCKS = 8              # the global snapshot block is 8 seeded row blocks, whatever the number of ranks
 EPS = float(np.finfo(np.float64).eps)
+# --dump-outputs: bytes per written array and its row list (60 MiB in all with the four reduced operators at r <= 512: under 64 MB)
+DUMP_CAP = {"gsm": 28 << 20, "q": 12 << 20, "info": 4 << 20}
+DUMP_CAP_OTHER = 4 << 20
 
 
 def workload_config(name, wl, n):
@@ -277,6 +282,28 @@ def measure_fp64_peak():
                              "MEASURED_PEAKS.json holds no FP64 figure and its bf16 figure does not bound an FP64 kernel")
 
 
+def dump_outputs(out_dir, arrays):
+    """Write every tensor of ``arrays`` as ``out_dir/<name>.npy`` in float64, complex ones with a trailing (real, imag) axis.  An
+    array above its byte cap keeps a sample of its leading-axis rows drawn with a fixed seed (the same rows on every run with the
+    same arguments), listed in ``<name>_rows.npy``."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if t is None:                                         # an all-zero operator is returned as None
+            continue
+        cap = DUMP_CAP.get(name, DUMP_CAP_OTHER)
+        row_bytes = max(1, t[0].numel()) * (16 if t.is_complex() else 8)
+        if t.shape[0] * row_bytes > cap:
+            keep = cap // (row_bytes + 8)                     # the row list counts against the cap too
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], keep, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+        a = t.cpu().numpy()
+        if np.iscomplexobj(a):
+            a = np.stack((a.real, a.imag), axis=-1)
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def make_path(wl_ops, rank, world):
     from scipy.constants import pi, epsilon_0
     from scipy.sparse import csc_array
@@ -395,6 +422,10 @@ def run_b200(args, name, wl, rank, world, local_rank):
     ms_step, out, launches = timed(step, args.steps, 0)
     clocks = sampler.stop()
     check_flags("timed loop")
+    if args.dump_outputs and rank == 0:
+        gsm_o, q_o, red_o, res_o = out
+        dump_outputs(args.dump_outputs, {"gsm": gsm_o, "q": q_o, "a0_r": red_o[0], "a1_r": red_o[1], "a2_r": red_o[2], "b_r": red_o[3],
+                                         "info": res_o.info})
     if use_graph:
         launches = args.steps * path.launches_per_graph          # a replay launches the captured kernels without passing the ABI counter
     value = f_total / (ms_step * 1e-3)
@@ -713,7 +744,16 @@ def main():
                          "valid because the synthetic operators and snapshots are real, like the reference's data)")
     ap.add_argument("--no-alt-dtype", action="store_true", help="skip the second timed loop on the other arithmetic type")
     ap.add_argument("--no-graph", action="store_true", help="run the eager (adaptive CholeskyQR) step instead of the CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (S-parameters, basis, reduced operators, per-point "
+                         "pivot info) as DIR/<name>.npy in float64, complex arrays with a trailing (real, imag) axis; a larger array "
+                         "keeps a fixed seeded sample of its rows (DIR/<name>_rows.npy), 64 MB in all.  With --gpus N > 1, rank 0 "
+                         "writes and the basis and pivot info are its own shard")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 path; the reference arm times a sample of the workload")
     wl = dict(WORKLOADS[args.workload])
     if args.r or args.points or args.ports:
         wl["r"], wl["f"], wl["m"] = args.r or wl["r"], args.points or wl["f"], args.ports or wl["m"]

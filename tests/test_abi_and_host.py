@@ -4,6 +4,9 @@ import ctypes
 import math
 import os
 import re
+import subprocess
+import sys
+import textwrap
 import warnings
 
 import numpy as np
@@ -74,13 +77,23 @@ def test_argument_validation_without_gpu():
 
 
 def test_product_path_refuses_to_run_without_cuda():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
-    a0, a1, a2, b = synthetic.reduced_model(8, 2, seed=0)
-    md = impl.ModelDefinition(np.linspace(3e9, 5e9, 4), a0, a1, a2, b, lambda t: 1.0, lambda t: t, lambda t: t ** 2, th.b_coefficient)
-    with pytest.raises(_ffi.MorfemB200Error):
-        impl.solve_finite_element_method(md)      # no CPU fallback on the hot path
+    """No CPU fallback on the hot path.  Runs in a child process with every GPU hidden, so that it checks the same thing on a
+    machine that has one."""
+    script = textwrap.dedent("""
+        import numpy as np, torch
+        from morfem_b200 import _ffi, implementation as impl, test_helpers as th, synthetic
+        assert not torch.cuda.is_available()
+        a0, a1, a2, b = synthetic.reduced_model(8, 2, seed=0)
+        md = impl.ModelDefinition(np.linspace(3e9, 5e9, 4), a0, a1, a2, b, lambda t: 1.0, lambda t: t, lambda t: t ** 2, th.b_coefficient)
+        try:
+            impl.solve_finite_element_method(md)
+        except _ffi.MorfemB200Error:
+            raise SystemExit(0)
+        raise SystemExit("solve_finite_element_method returned without a CUDA device")
+    """)
+    out = subprocess.run([sys.executable, "-c", script], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True,
+                         text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
 
 
 def test_b_coefficient_scalar_and_array_forms_agree():

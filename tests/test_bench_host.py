@@ -58,3 +58,28 @@ def test_snapshot_block_does_not_depend_on_the_rank_count():
             parts.append(b.snapshot_rows(n, r, lo, hi))
         assert np.array_equal(np.concatenate(parts, axis=0), whole)                  # bit-identical global problem at every N
     assert np.linalg.matrix_rank(whole) == r
+
+
+def test_dump_outputs_float64_capped_and_seeded(tmp_path, monkeypatch):
+    """--dump-outputs: float64 files, complex arrays with a trailing (real, imag) axis, no file for an all-zero (None) operator, an
+    array over its cap cut to a sorted seeded sample of its rows (the same rows on every run), 64 MB in all at the default caps."""
+    import torch
+    b = _bench()
+    assert sum(b.DUMP_CAP.values()) + 4 * b.DUMP_CAP_OTHER <= 64e6          # gsm, q, info and the four reduced operators
+    monkeypatch.setitem(b.DUMP_CAP, "gsm", 1 << 16)
+    gsm = torch.randn(10000, 2, 2, dtype=torch.complex128)
+    q = torch.randn(300, 8, dtype=torch.float64)
+    info = torch.arange(10000, dtype=torch.int32)
+    for d in ("a", "b"):
+        b.dump_outputs(str(tmp_path / d), {"gsm": gsm, "q": q, "a1_r": None, "info": info})
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["gsm.npy", "gsm_rows.npy", "info.npy", "q.npy"]
+    for name in names:
+        x = np.load(tmp_path / "a" / name)
+        assert x.dtype == np.float64 and np.array_equal(x, np.load(tmp_path / "b" / name))
+    rows = np.load(tmp_path / "a" / "gsm_rows.npy").astype(np.int64)
+    g = np.load(tmp_path / "a" / "gsm.npy")
+    assert g.shape == (rows.size, 2, 2, 2) and g.nbytes + rows.nbytes <= 1 << 16 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(g[..., 0] + 1j * g[..., 1], gsm.numpy()[rows])
+    assert np.array_equal(np.load(tmp_path / "a" / "q.npy"), q.numpy())
+    assert np.array_equal(np.load(tmp_path / "a" / "info.npy"), np.arange(10000.0))
