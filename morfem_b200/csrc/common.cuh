@@ -70,6 +70,20 @@ __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double
                  : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
+// Complex 8x8x4 block product in Gauss's three-multiplication form ("3M", as in ZGEMM3M): three real DMMAs instead of four.
+// With a = ar + i ai (A fragment) and b = br + i bi (B fragment), three accumulator planes take
+//   k1 += (ar + ai) br,   k2 += ar (bi - br),   k3 += ai (br + bi),   and then   re = k1 - k3,   im = k1 + k2.
+// The operand combinations are formed once per fragment and reused by every tile the fragment feeds.  On real data embedded in
+// complex128 (ai = bi = 0) k1 is the same DMMA sequence as the real plane of the four-product form, k2 = -k1 and k3 = 0 exactly, so
+// re is bit-identical to it and im is exactly zero.  On complex data the error stays normwise of order k eps |A| |B| with a somewhat
+// larger constant than the four-product form.
+__device__ __forceinline__ void cmma3(double (&k1)[2], double (&k2)[2], double (&k3)[2], double ar, double ai, double as,
+                                      double br, double bd, double bs) {
+    dmma884(k1[0], k1[1], as, br);
+    dmma884(k2[0], k2[1], ar, bd);
+    dmma884(k3[0], k3[1], ai, bs);
+}
+
 // Ampere-style async copy, 16 bytes, global -> shared (SASS LDGSTS), with zero-fill predicate.
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src, bool valid) {
     unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);

@@ -5,8 +5,12 @@
 //             matrices of the CholeskyQR2 replacement of np.linalg.svd (implementation.py:226/298/210).
 //   gemm_nn : Out (n x rb) = A (n x ra) W (ra x rb): the `S R^-1` and `Q1 (R2^-1 U)` applications.
 //
-// Complex data stays interleaved: one 16-byte shared-memory load yields the (re, im) pair that feeds the four
-// real DMMAs of a complex 8x8x4 block product.  Operand tiles are staged with cp.async (LDGSTS) in a 3-stage
+// Complex data stays interleaved: one 16-byte shared-memory load yields the (re, im) pair of a fragment.  Each complex
+// 8x8x4 block product is three real DMMAs in Gauss's form (cmma3, common.cuh) instead of four: a warp forms the operand
+// combinations of a fragment once (one DADD per A fragment, two per B fragment) and reuses them across its warp tile, and
+// the three accumulator planes are combined into (re, im) in the epilogue.  Three planes of a 32 x 32 warp tile would not
+// fit the register file next to the fragments, so a warp owns 32 x 16 (96 accumulator registers) and the CTAs have twice
+// the warps of the four-product kernels at the same CTA tile.  Operand tiles are staged with cp.async (LDGSTS) in a 3-stage
 // ring; shared-memory leading dimensions are padded so every quarter-warp fragment load is conflict-free.
 // Roofline: FP64 tensor pipe (37.05 TFLOP/s measured, tools/fp64_peaks.cu) for r >~ 48, HBM below that.
 #include "common.cuh"
@@ -17,17 +21,20 @@ constexpr int KC = 16;        // rows of the reduction index per pipeline stage
 constexpr int STAGES = 3;
 
 // ------------------------------------------------------------------------------------------------ gemm_tn
-constexpr int TN_TI = 64, TN_TJ = 64, TN_THREADS = 128;
+constexpr int TN_TI = 64, TN_TJ = 64, TN_THREADS = 256;      // 2 x 4 warps, each 32 x 16
 constexpr int TN_LDA = TN_TI + 2, TN_LDB = TN_TJ + 2;        // == 2 (mod 8) complex -> conflict-free fragments
 constexpr int TN_STAGE_ELEMS = KC * (TN_LDA + TN_LDB);
 
-__global__ void __launch_bounds__(TN_THREADS, 2)
+// CONJ: C = A^H B.  With a = ar - i ai the 3M planes are k1 += (ar - ai) br and k3 += ai (br + bi) with re = k1 + k3, so no operand
+// is negated in the loop.
+template <bool CONJ>
+__global__ void __launch_bounds__(TN_THREADS, 2)      // <= 128 registers: two CTAs (16 warps) per SM
 gemm_tn_kernel(const cplx* __restrict__ A, long long lda, int ra, const cplx* __restrict__ B, long long ldb, int rb,
-               long long n, long long rows_per_split, int conj_a, cplx* __restrict__ part, int herm) {
+               long long n, long long rows_per_split, cplx* __restrict__ part, int herm) {
     extern __shared__ __align__(16) cplx smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int g = lane >> 2, t = lane & 3;
-    const int wi = warp >> 1, wj = warp & 1;
+    const int wi = warp >> 2, wj = warp & 3;
     const int ntj = (rb + TN_TJ - 1) / TN_TJ;
     const int ti = blockIdx.x / ntj, tj = blockIdx.x - ti * ntj;
     if (herm && ti > tj) return;               // Gram matrix A^H A: the lower tiles are the conjugate transposes of the upper ones
@@ -60,14 +67,15 @@ gemm_tn_kernel(const cplx* __restrict__ A, long long lda, int ra, const cplx* __
         }
     };
 
-    double cre[4][4][2], cim[4][4][2];
+    double k1[4][2][2], k2[4][2][2], k3[4][2][2];            // the three 3M planes of a 4 x 2 grid of 8 x 8 tiles
 #pragma unroll
     for (int i = 0; i < 4; ++i)
 #pragma unroll
-        for (int j = 0; j < 4; ++j) { cre[i][j][0] = cre[i][j][1] = 0.0; cim[i][j][0] = cim[i][j][1] = 0.0; }
+        for (int j = 0; j < 2; ++j)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) k1[i][j][e] = k2[i][j][e] = k3[i][j][e] = 0.0;
 
     for (int s = 0; s < STAGES - 1; ++s) { if (s < nchunks) load_stage(s, s); cp_async_commit(); }
-    const double sgn = conj_a ? -1.0 : 1.0;
     for (int c = 0; c < nchunks; ++c) {
         cp_async_wait<STAGES - 2>();
         __syncthreads();
@@ -76,34 +84,36 @@ gemm_tn_kernel(const cplx* __restrict__ A, long long lda, int ra, const cplx* __
         const cplx* Bs = As + KC * TN_LDA;
 #pragma unroll
         for (int kk = 0; kk < KC / 4; ++kk) {
-            cplx a[4], b[4];
+            double br[2], bd[2], bs[2];
 #pragma unroll
-            for (int i = 0; i < 4; ++i) { a[i] = As[(kk * 4 + t) * TN_LDA + wi * 32 + i * 8 + g]; a[i].y *= sgn; }
+            for (int j = 0; j < 2; ++j) {
+                const cplx b = Bs[(kk * 4 + t) * TN_LDB + wj * 16 + j * 8 + g];
+                br[j] = b.x; bd[j] = b.y - b.x; bs[j] = b.x + b.y;
+            }
 #pragma unroll
-            for (int j = 0; j < 4; ++j) b[j] = Bs[(kk * 4 + t) * TN_LDB + wj * 32 + j * 8 + g];
+            for (int i = 0; i < 4; ++i) {
+                const cplx a = As[(kk * 4 + t) * TN_LDA + wi * 32 + i * 8 + g];
+                const double as = CONJ ? a.x - a.y : a.x + a.y;
 #pragma unroll
-            for (int i = 0; i < 4; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    dmma884(cre[i][j][0], cre[i][j][1], a[i].x, b[j].x);
-                    dmma884(cre[i][j][0], cre[i][j][1], -a[i].y, b[j].y);
-                    dmma884(cim[i][j][0], cim[i][j][1], a[i].x, b[j].y);
-                    dmma884(cim[i][j][0], cim[i][j][1], a[i].y, b[j].x);
-                }
+                for (int j = 0; j < 2; ++j) cmma3(k1[i][j], k2[i][j], k3[i][j], a.x, a.y, as, br[j], bd[j], bs[j]);
+            }
         }
     }
     cp_async_wait<0>();
-    // partial tile -> part[split][ra][rb]
+    // partial tile -> part[split][ra][rb]; the planes are combined here, so the split-K summation sees (re, im) as before
     cplx* out = part + (long long)blockIdx.y * ra * rb;
 #pragma unroll
     for (int i = 0; i < 4; ++i)
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
+        for (int j = 0; j < 2; ++j) {
             int row = i0 + wi * 32 + i * 8 + g;
-            int col = j0 + wj * 32 + j * 8 + 2 * t;
+            int col = j0 + wj * 16 + j * 8 + 2 * t;
             if (row < ra) {
-                if (col < rb) out[(long long)row * rb + col] = cmake(cre[i][j][0], cim[i][j][0]);
-                if (col + 1 < rb) out[(long long)row * rb + col + 1] = cmake(cre[i][j][1], cim[i][j][1]);
+#pragma unroll
+                for (int e = 0; e < 2; ++e)
+                    if (col + e < rb)
+                        out[(long long)row * rb + col + e] = cmake(CONJ ? k1[i][j][e] + k3[i][j][e] : k1[i][j][e] - k3[i][j][e],
+                                                                   k1[i][j][e] + k2[i][j][e]);
             }
         }
 }
@@ -161,18 +171,18 @@ void tn_plan(int ra, int rb, long long n, int& tiles, int& nsplit, long long& ro
 }
 
 // ------------------------------------------------------------------------------------------------ gemm_nn
-constexpr int NN_TM = 128, NN_TN = 64, NN_THREADS = 256;
+constexpr int NN_TM = 128, NN_TN = 64, NN_THREADS = 512;     // 4 x 4 warps, each 32 x 16
 constexpr int NN_LDA = KC + 4;          // == 4 (mod 8): A-fragment (row g, col t) loads conflict-free
 constexpr int NN_LDW = NN_TN + 2;
 constexpr int NN_STAGE_ELEMS = NN_TM * NN_LDA + KC * NN_LDW;
 
-__global__ void __launch_bounds__(NN_THREADS, 1)
+__global__ void __launch_bounds__(NN_THREADS, 1)      // <= 128 registers: one 16-warp CTA per SM
 gemm_nn_kernel(const cplx* __restrict__ A, long long lda, long long n, int ra, const cplx* __restrict__ W, long long ldw, int rb,
                cplx* __restrict__ Out, long long ldo, int w_upper) {
     extern __shared__ __align__(16) cplx smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int g = lane >> 2, t = lane & 3;
-    const int wm = warp >> 1, wn = warp & 1;          // 4 x 2 warps, each 32 x 32
+    const int wm = warp >> 2, wn = warp & 3;          // 4 x 4 warps, each 32 x 16
     const int ntn = (rb + NN_TN - 1) / NN_TN;
     const long long tm = blockIdx.x / ntn; const int tn = (int)(blockIdx.x - tm * ntn);
     const long long m0 = tm * NN_TM; const int j0 = tn * NN_TN;
@@ -180,17 +190,24 @@ gemm_nn_kernel(const cplx* __restrict__ A, long long lda, long long n, int ra, c
     const int kmax = (w_upper && j0 + NN_TN < ra) ? j0 + NN_TN : ra;
     const int nchunks = (kmax + KC - 1) / KC;
 
+    // A rows of this thread: tid / KC + q NN_THREADS / KC, column tid % KC of every chunk (row pointer and bounds fixed once:
+    // the 16-warp CTA runs at the 128-register cap)
+    constexpr int NN_AQ = (NN_TM * KC) / NN_THREADS, NN_AROWS = NN_THREADS / KC;
+    const int a_rr = tid / KC, a_cc = tid - a_rr * KC;
+    const cplx* a_src = A + (m0 + a_rr) * lda + a_cc;
+    unsigned a_rows_ok = 0;
+#pragma unroll
+    for (int q = 0; q < NN_AQ; ++q) a_rows_ok |= (m0 + a_rr + q * NN_AROWS < n) ? 1u << q : 0u;
+
     auto load_stage = [&](int stage, int chunk) {
         cplx* As = smem + stage * NN_STAGE_ELEMS;
         cplx* Ws = As + NN_TM * NN_LDA;
         const int k0 = chunk * KC;
 #pragma unroll
-        for (int q = 0; q < (NN_TM * KC) / NN_THREADS; ++q) {
-            int idx = tid + q * NN_THREADS;
-            int rr = idx / KC, cc = idx - rr * KC;
-            bool ok = (m0 + rr) < n && (k0 + cc) < ra;
-            const cplx* src = A + (ok ? (m0 + rr) * lda + k0 + cc : 0);
-            cp_async16(As + rr * NN_LDA + cc, src, ok);
+        for (int q = 0; q < NN_AQ; ++q) {
+            const bool ok = ((a_rows_ok >> q) & 1u) && (k0 + a_cc) < ra;
+            const cplx* src = ok ? a_src + q * NN_AROWS * lda + k0 : A;
+            cp_async16(As + (a_rr + q * NN_AROWS) * NN_LDA + a_cc, src, ok);
         }
 #pragma unroll
         for (int q = 0; q < (KC * NN_TN) / NN_THREADS; ++q) {
@@ -202,11 +219,13 @@ gemm_nn_kernel(const cplx* __restrict__ A, long long lda, long long n, int ra, c
         }
     };
 
-    double cre[4][4][2], cim[4][4][2];
+    double k1[4][2][2], k2[4][2][2], k3[4][2][2];            // the three 3M planes of a 4 x 2 grid of 8 x 8 tiles
 #pragma unroll
     for (int i = 0; i < 4; ++i)
 #pragma unroll
-        for (int j = 0; j < 4; ++j) { cre[i][j][0] = cre[i][j][1] = 0.0; cim[i][j][0] = cim[i][j][1] = 0.0; }
+        for (int j = 0; j < 2; ++j)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) k1[i][j][e] = k2[i][j][e] = k3[i][j][e] = 0.0;
 
     for (int s = 0; s < STAGES - 1; ++s) { if (s < nchunks) load_stage(s, s); cp_async_commit(); }
     for (int c = 0; c < nchunks; ++c) {
@@ -217,38 +236,39 @@ gemm_nn_kernel(const cplx* __restrict__ A, long long lda, long long n, int ra, c
         const cplx* Ws = As + NN_TM * NN_LDA;
 #pragma unroll
         for (int kk = 0; kk < KC / 4; ++kk) {
-            cplx a[4], b[4];
+            double br[2], bd[2], bs[2];
 #pragma unroll
-            for (int i = 0; i < 4; ++i) a[i] = As[(wm * 32 + i * 8 + g) * NN_LDA + kk * 4 + t];
+            for (int j = 0; j < 2; ++j) {
+                const cplx b = Ws[(kk * 4 + t) * NN_LDW + wn * 16 + j * 8 + g];
+                br[j] = b.x; bd[j] = b.y - b.x; bs[j] = b.x + b.y;
+            }
 #pragma unroll
-            for (int j = 0; j < 4; ++j) b[j] = Ws[(kk * 4 + t) * NN_LDW + wn * 32 + j * 8 + g];
+            for (int i = 0; i < 4; ++i) {
+                const cplx a = As[(wm * 32 + i * 8 + g) * NN_LDA + kk * 4 + t];
+                const double as = a.x + a.y;
 #pragma unroll
-            for (int i = 0; i < 4; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    dmma884(cre[i][j][0], cre[i][j][1], a[i].x, b[j].x);
-                    dmma884(cre[i][j][0], cre[i][j][1], -a[i].y, b[j].y);
-                    dmma884(cim[i][j][0], cim[i][j][1], a[i].x, b[j].y);
-                    dmma884(cim[i][j][0], cim[i][j][1], a[i].y, b[j].x);
-                }
+                for (int j = 0; j < 2; ++j) cmma3(k1[i][j], k2[i][j], k3[i][j], a.x, a.y, as, br[j], bd[j], bs[j]);
+            }
         }
     }
     cp_async_wait<0>();
 #pragma unroll
     for (int i = 0; i < 4; ++i)
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
+        for (int j = 0; j < 2; ++j) {
             long long row = m0 + wm * 32 + i * 8 + g;
-            int col = j0 + wn * 32 + j * 8 + 2 * t;
+            int col = j0 + wn * 16 + j * 8 + 2 * t;
+            const double re0 = k1[i][j][0] - k3[i][j][0], im0 = k1[i][j][0] + k2[i][j][0];
+            const double re1 = k1[i][j][1] - k3[i][j][1], im1 = k1[i][j][1] + k2[i][j][1];
             if (row < n) {
                 if (col + 1 < rb) {
                     // two adjacent complex elements: 32 contiguous bytes
-                    double4 v = make_double4(cre[i][j][0], cim[i][j][0], cre[i][j][1], cim[i][j][1]);
+                    double4 v = make_double4(re0, im0, re1, im1);
                     cplx* dst = Out + row * ldo + col;
                     if ((reinterpret_cast<uintptr_t>(dst) & 31) == 0) *reinterpret_cast<double4*>(dst) = v;
                     else { dst[0] = cmake(v.x, v.y); dst[1] = cmake(v.z, v.w); }
                 } else if (col < rb) {
-                    Out[row * ldo + col] = cmake(cre[i][j][0], cim[i][j][0]);
+                    Out[row * ldo + col] = cmake(re0, im0);
                 }
             }
         }
@@ -278,9 +298,10 @@ extern "C" int mf_gemm_tn_c128(const mf_c128* A, int64_t lda, int ra, const mf_c
     const int herm = (conj_a && (const void*)A == (const void*)B && lda == ldb && ra == rb) ? 1 : 0;
     tn_plan(ra, rb, n > 0 ? n : 1, tiles, nsplit, rps, herm != 0);
     const size_t smem = sizeof(cplx) * STAGES * TN_STAGE_ELEMS;
-    MF_CHECK_CUDA(cudaFuncSetAttribute(gemm_tn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    auto kern = conj_a ? gemm_tn_kernel<true> : gemm_tn_kernel<false>;
+    MF_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     dim3 grid(tiles, nsplit);
-    gemm_tn_kernel<<<grid, TN_THREADS, smem, st>>>((const cplx*)A, lda, ra, (const cplx*)B, ldb, rb, n, rps, conj_a, (cplx*)ws, herm);
+    kern<<<grid, TN_THREADS, smem, st>>>((const cplx*)A, lda, ra, (const cplx*)B, ldb, rb, n, rps, (cplx*)ws, herm);
     MF_CHECK_LAUNCH();
     long long total = (long long)ra * rb;
     reduce_partials_kernel<<<(unsigned)((total + 31) / 32), RED_WARPS * 32, 0, st>>>((const cplx*)ws, nsplit, ra, rb, (cplx*)C, ldc, herm);

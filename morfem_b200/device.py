@@ -173,6 +173,8 @@ def gemm_tn(a: torch.Tensor, b: torch.Tensor, conj: bool = False, out: Optional[
         return out
     nbytes = lib.mf_gemm_tn_ws_bytes(ra, rb, n)
     ws = workspaces.get("gemm_tn", nbytes, a.device)
+    # complex flops are counted as the algorithmic 8 n ra rb (four real products per complex one) although the kernels issue three
+    # (Gauss's form, dense_gemm.cu): TFLOP/s and shares of peak stay comparable with the four-product kernels
     with _timed("gemm_tn", nbytes=16.0 * n * (ra if same else ra + rb) + 16.0 * ra * rb, flops=8.0 * n * ra * rb):
         _ffi.check(lib.mf_gemm_tn_c128(_ptr(a), a.stride(0), ra, _ptr(b), b.stride(0), rb, n, int(conj), _ptr(out), out.stride(0),
                                        _ptr(ws), ws.numel(), _stream()), "mf_gemm_tn_c128")
