@@ -6,9 +6,9 @@ Models.  A seeded reduced waveguide model (``synthetic.reduced_model``) with a l
 and 1e-6), near-real (|Im| ~ 1e-9 |Re|: the kernels must not take their real fast paths) and near-imaginary (the same model times i:
 pivots that are almost purely imaginary).  The loss sets how close the points come to a resonance: cond2(A(t)) runs from ~1e3 to ~1e7.
 
-Reference.  Per point, A(t) = c0 A0 + c1 A1 + c2 A2 from the same symmetrised operators the kernels receive, solved by zgetrf
-(scipy ``lu_factor`` / ``lu_solve``) and two steps of iterative refinement with the residual in clongdouble: x*.  S* = 2 (I + Z*^-1)^-1 - I
-with Z* = j zs x*^T (cb Br).  The unrefined zgetrf solution must pass the same checks before x* is used, so that a failure points at
+Reference (``sweep_reference``).  Per point, A(t) = c0 A0 + c1 A1 + c2 A2 from the same symmetrised operators the kernels receive,
+solved by zgetrf (scipy ``lu_factor`` / ``lu_solve``) and two steps of iterative refinement with the residual in clongdouble: x*.
+S* = 2 (I + Z*^-1)^-1 - I with Z* = j zs x*^T (cb Br).  The unrefined zgetrf solution must pass the same checks before x* is used, so that a failure points at
 the kernel and not at the test.
 
 Checks (LAPACK's test ratios, with the threshold 30 of its zchkge suite):
@@ -24,41 +24,21 @@ import os
 import subprocess
 import sys
 import textwrap
-from collections import defaultdict
 
 import numpy as np
 import pytest
-from scipy.constants import epsilon_0, pi
-from scipy.linalg import lapack, lu_factor, lu_solve
+from scipy.linalg import lapack
 
 torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
-from oracle import reference_path as orc   # noqa: E402  (checker only)
+from sweep_reference import (EPS, SWITCHES, THRESH, WORST, Reference, check, coefficients, complex_model, frequencies,  # noqa: E402,F401
+                             gsm_host, real_model, report, sample, set_switches, singular_block, singular_columns, symmetrised)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EPS = np.finfo(np.float64).eps
-THRESH = 30.0
-CLD = np.clongdouble
-
-# the switches the sweep reads on every call; each run sets exactly the ones it names and clears the others
-SWITCHES = ("MF_LEFT_VER", "MF_LEFT_CFG", "MF_LEFT_CHUNK", "MF_LEFT_LOOKAHEAD", "MF_STREAM_CFG", "MF_STREAM_FUSE",
-            "MF_SWEEP_FORCE_SMEM", "MF_SWEEP_FORCE_LEFT")
 
 # (regime, relative loss)
 MODELS = (("balanced", 1e-2), ("balanced", 1e-6), ("near_real", 1e-9), ("near_imag", 1e-9))
-
-WORST = defaultdict(lambda: np.zeros(3))      # family -> largest (backward, forward, S) ratio
-
-
-@pytest.fixture(scope="module", autouse=True)
-def report():
-    yield
-    if WORST:
-        print("\nlargest ratios per family (threshold %g):  backward  forward  S" % THRESH)
-        for fam in sorted(WORST):
-            b, f, s = WORST[fam]
-            print(f"  {fam:<22s} {b:9.3f} {f:8.3f} {s:8.3f}")
 
 
 @pytest.fixture(scope="module")
@@ -72,146 +52,6 @@ def dv():
 def lib():
     from morfem_b200 import _ffi
     return _ffi.load()
-
-
-# ------------------------------------------------------------------------------------------------------------ models
-def complex_model(regime, loss, r, m):
-    """Host operators ``[a0, a1, a2]`` (complex, not symmetrised) and the port matrix ``br`` (r x m, complex)."""
-    from morfem_b200 import synthetic
-    seed = 1000 + 7 * r + m
-    a0, _, a2, b = synthetic.reduced_model(r, m, seed=seed)
-    rng = np.random.default_rng(seed)
-
-    def sym():                                              # symmetric, 2-norm ~ 1
-        g = rng.standard_normal((r, r))
-        return (g + g.T) / (2.0 * np.sqrt(2.0 * r))
-
-    n0, n2 = np.abs(a0).max(), np.abs(a2).max()
-    a1 = (sym() + 1j * loss * sym()) * 1e-3 * n0 / 4e9       # c1(t) = t: a conductor-like term, 1e-3 of a0 at 4 GHz
-    a0 = a0 + 1j * loss * n0 * sym()
-    a2 = a2 + 1j * loss * n2 * sym()
-    b2 = rng.standard_normal(b.shape) * np.sqrt(np.mean(b ** 2))
-    phase, bre, bim = {"balanced": (np.exp(0.6j), 1.0, 1.0), "near_real": (1.0, 1.0, 1e-9), "near_imag": (1j, 1e-9, 1.0)}[regime]
-    return [phase * a for a in (a0, a1, a2)], bre * b + 1j * bim * b2
-
-
-def real_model(r, m):
-    from morfem_b200 import synthetic
-    a0, _, a2, b = synthetic.reduced_model(r, m, seed=2000 + r)
-    rng = np.random.default_rng(r)
-    g = rng.standard_normal((r, r))
-    a1 = 1e-3 * np.abs(a0).max() / 4e9 * (g + g.T) / (2.0 * np.sqrt(2.0 * r))
-    return [a0.astype(complex), a1.astype(complex), a2.astype(complex)], b.astype(complex)
-
-
-def singular_block(r, k):
-    """Identity with the symmetric block [[2+2i, 1+i], [1+i, 0.5+0.5i]] at rows/columns k, k+1: under |re|+|im| pivoting the multiplier is
-    exactly 0.5 and U[k+1, k+1] exactly 0, so LU reports info = k + 2."""
-    a = np.eye(r, dtype=complex)
-    a[k:k + 2, k:k + 2] = [[2 + 2j, 1 + 1j], [1 + 1j, 0.5 + 0.5j]]
-    return a
-
-
-def frequencies(nf):
-    return np.array([4e9]) if nf == 1 else np.linspace(3e9, 5e9, nf)
-
-
-def coefficients(f):
-    """(c0, c1, c2, cb, zs) of the waveguide sweep at the points f."""
-    return np.ones_like(f), f.copy(), f ** 2, np.array([orc.b_coefficient(t) for t in f]), 2 * pi * f * epsilon_0
-
-
-def symmetrised(ops):
-    return [None if a is None else (a + a.T) / 2 for a in ops]
-
-
-# --------------------------------------------------------------------------------------------------------- reference
-def system(sops, coef, i, dtype=complex):
-    a = None
-    for c, s in zip(coef[:3], sops):
-        if s is not None:
-            t = dtype(c[i]) * s.astype(dtype, copy=False)
-            a = t if a is None else a + t
-    return a
-
-
-def cond2(a):
-    s = np.linalg.svd(a, compute_uv=False)
-    return s[0] / s[-1]
-
-
-def sample(nf, r, extra=()):
-    n = min(nf, 16 if r <= 256 else (8 if r <= 512 else 3))
-    return np.unique(np.concatenate([np.linspace(0, nf - 1, n).round().astype(int), np.asarray(extra, dtype=int)]))
-
-
-def backward_ratios(sops, coef, br, x):
-    """Per point: max over the right-hand sides of ||b - A x||_1 / (r ||A||_1 ||x||_1 eps), the residual in clongdouble."""
-    nf, r, m = x.shape
-    xl = np.moveaxis(x, 0, 1).reshape(r, nf * m).astype(CLD)
-    res = (coef[3][:, None, None] * br[None].astype(CLD)).astype(CLD)
-    for c, s in zip(coef[:3], sops):
-        if s is not None:
-            res = res - c[:, None, None] * np.moveaxis((s.astype(CLD) @ xl).reshape(r, nf, m), 1, 0)
-    rn = np.abs(res).sum(axis=1).astype(np.float64)                                   # (nf, m) column 1-norms
-    xn = np.abs(x).sum(axis=1)
-    an = np.array([np.abs(system(sops, coef, i)).sum(axis=0).max() for i in range(nf)])
-    with np.errstate(divide="ignore", invalid="ignore"):
-        return np.max(rn / (r * an[:, None] * xn * EPS), axis=1)
-
-
-def gsm_host(x, br, cb, zs):
-    z = 1j * zs * (x.T @ (cb * br))
-    ident = np.eye(z.shape[0])
-    return z, 2 * np.linalg.inv(ident + np.linalg.inv(z)) - ident
-
-
-class Reference:
-    """The refined reference of one model at the points ``idx`` of a coefficient set (x*, cond2, S*, kappa per point)."""
-
-    def __init__(self, sops, br, coef, idx):
-        self.sops, self.br, self.coef, self.idx = sops, br, coef, np.asarray(idx)
-        r, m = br.shape
-        self.has_s = m <= r            # for m > r, Z = j zs x^T B has rank r < m: no S-parameters to compare
-        self.xs, self.cond, self.ss, self.kappa, x0s = [], [], [], [], []
-        for i in self.idx:
-            a, al = system(sops, coef, i), system(sops, coef, i, CLD)
-            b = coef[3][i] * br
-            lu = lu_factor(a)
-            x0 = lu_solve(lu, b)
-            xl = x0.astype(CLD)
-            for _ in range(2):
-                xl = xl + lu_solve(lu, (b.astype(CLD) - al @ xl).astype(complex))
-            xs = xl.astype(complex)
-            c = cond2(a)
-            self.xs.append(xs); self.cond.append(c); x0s.append(x0)
-            if self.has_s:
-                bb = coef[3][i] * br
-                z, s = gsm_host(xs, br, coef[3][i], coef[4][i])
-                self.ss.append(s)
-                self.kappa.append(c * np.linalg.norm(xs, 2) * np.linalg.norm(bb, 2) / np.linalg.norm(xs.T @ bb, 2) * np.linalg.cond(z) *
-                                  np.linalg.cond(np.eye(m) + np.linalg.inv(z)))
-        self.xs, self.ss = np.array(self.xs), np.array(self.ss)
-        self.cond, self.kappa = np.array(self.cond), np.array(self.kappa)
-        # zgetrf's own solution must pass every check against x* (else the reference could not tell a kernel error)
-        x0s = np.array(x0s)
-        sub = [c[self.idx] for c in coef]
-        assert np.all(backward_ratios(sops, sub, br, x0s) < THRESH)
-        assert np.all(self.forward(x0s) < THRESH)
-        if self.has_s:
-            s0 = np.array([gsm_host(x0, br, coef[3][i], coef[4][i])[1] for x0, i in zip(x0s, self.idx)])
-            assert np.all(self.s_ratios(s0) < THRESH)
-
-    def forward(self, x):
-        """||x - x*||_F / (||x*||_F cond2(A) eps) at the reference points (x indexed like ``idx``)."""
-        d = np.linalg.norm((x - self.xs).reshape(len(self.idx), -1), axis=1)
-        return d / (np.linalg.norm(self.xs.reshape(len(self.idx), -1), axis=1) * self.cond * EPS)
-
-    def s_ratios(self, s):
-        if not self.has_s:
-            return np.zeros(1)
-        d = np.linalg.norm((s - self.ss).reshape(len(self.idx), -1), axis=1)
-        return d / (np.linalg.norm(self.ss.reshape(len(self.idx), -1), axis=1) * self.kappa * EPS)
 
 
 _models, _refs, _dev = {}, {}, {}
@@ -240,34 +80,11 @@ def device_operands(dv, key, r, m):
     return _dev[(key, r, m)]
 
 
-def set_switches(monkeypatch, env):
-    for k in SWITCHES:
-        if k in env and env[k] is not None:
-            monkeypatch.setenv(k, str(env[k]))
-        else:
-            monkeypatch.delenv(k, raising=False)
-
-
 def run_sweep(dv, dops, dbr, coef, variant, want_gsm=True):
     t = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).cuda()  # noqa: E731
     res = dv.sweep(*dops, dbr, *(t(c) for c in coef), want_x=True, want_gsm=want_gsm, variant=variant)
     torch.cuda.synchronize()
     return res.x.cpu().numpy(), (res.gsm.cpu().numpy() if want_gsm else None), res.info.cpu().numpy()
-
-
-def check(family, ref, x, s, info, points=None):
-    """Every check of the module on one run; ``points`` restricts the backward error to a subset (default: all)."""
-    points = np.arange(x.shape[0]) if points is None else np.asarray(points)
-    assert not np.any(info[points]), (family, np.flatnonzero(info))
-    coef = [c[points] for c in ref.coef]
-    bw = backward_ratios(ref.sops, coef, ref.br, x[points])
-    fw = ref.forward(x[ref.idx])
-    sr = ref.s_ratios(s[ref.idx])
-    w = WORST[family]
-    w[:] = np.maximum(w, [bw.max(), fw.max(), sr.max()])
-    assert np.all(bw < THRESH), (family, "backward", bw.max(), int(points[np.argmax(bw)]))
-    assert np.all(fw < THRESH), (family, "forward", fw.max(), int(ref.idx[np.argmax(fw)]))
-    assert np.all(sr < THRESH), (family, "S", sr.max(), int(ref.idx[np.argmax(sr)]))
 
 
 # ------------------------------------------------------------------------------------------------ families and cases
@@ -404,12 +221,6 @@ def test_rotation_by_i_and_conjugation(dv, monkeypatch, family, r, m):
     cj = _pair_ratio(xc, x.conj(), cplx)
     assert np.all(cj < THRESH), ("conjugation", cj.max())
     WORST[family][1] = max(WORST[family][1], rot.max(), cj.max())
-
-
-def singular_columns(r):
-    """k such that columns k, k+1 straddle an 8-column register panel, a 16-column block column and a deep panel."""
-    deep = 16 * ((r - 1) // 16) - 1
-    return sorted({k for k in (7, 15, deep - 8, deep) if 0 <= k and k + 1 < r})
 
 
 @pytest.mark.parametrize("family,r,m", PROPERTY_CASES)
